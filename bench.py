@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — MBAR self-consistent iteration throughput on B200 (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json metric / configs[2] shape): synthetic harmonic-oscillator u_kn, K = 256
 states, N = 1e7 samples PER GPU (20.48 GB of fp64 in HBM, far larger than the 126 MB L2), equal N_k,
@@ -190,6 +190,7 @@ def time_c_port(K, n_sample=400_000):
     try:
         from oracle import c_oracle
 
+        c_oracle.load(build=False)           # built by build(); the benchmark compiles nothing into the tree
         u, N_k = cpu_sample(K, n_sample)
         f = np.zeros(K)
         c_oracle.self_consistent_update(u, N_k, f)
@@ -736,6 +737,10 @@ def run_ours(args):
     loop = prob.last_loop_ms()                             # CUDA events on the launching stream
     rig.barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives: f_k after the last step (identical on every rank)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "f_k.npy"), np.asarray(f, dtype=np.float64))
     c1 = prob.counters()
     kernel_desc = prob.last_kernels()["pass_kernel"]      # the variant that actually ran in the timed loop
 
@@ -898,7 +903,14 @@ def main():
     ap.add_argument("--no-extra-configs", dest="extra_configs", action="store_false")
     ap.add_argument("--no-c5-hessian", dest="c5_hessian", action="store_false")
     ap.add_argument("--cpu-budget", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write f_k after the last timed step as DIR/f_k.npy (float64; c3 workload of --impl ours); "
+                         "the seeded inputs make it comparable between builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "c3"):
+        ap.error("--dump-outputs applies to the default workload (--impl ours --config c3)")
     args.warmup = max(args.warmup, 3)
     world = env_int("WORLD_SIZE", 1)
     if args.gpus > 1 and world == 1 and args.impl == "ours":

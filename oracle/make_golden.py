@@ -169,10 +169,23 @@ def c1_case():
     np.savez_compressed(path, **data)
 
 
+def bar_init_case():
+    """MBAR._initialize_with_bar (mbar.py:1936-1988) on an empty-state harmonic sample: what tests/test_initialize.py
+    compares pymbar_b200.initialize with."""
+    tc = ref_ts.harmonic_oscillators.HarmonicOscillatorsTestCase(O_k=[0, 1, 2, 3, 4], K_k=[1, 2, 4, 8, 16])
+    _, u, N, _ = tc.sample([300, 200, 0, 250, 100], mode="u_kn", seed=3)
+    m = pymbar.MBAR(u, N, initialize="zeros")
+    np.savez_compressed(os.path.join(OUT, "bar_init_5.npz"), u_kn=np.array(m.u_kn), N_k=np.array(m.N_k),
+                        x_kindices=np.array(m.x_kindices), f_bar=np.array(m._initialize_with_bar(m.u_kn)))
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     if "--only-c1" in sys.argv:
         c1_case()
+        return
+    if "--only-bar-init" in sys.argv:
+        bar_init_case()
         return
     rng = np.random.RandomState(1234)
 

@@ -141,6 +141,18 @@ def test_default_line_has_every_key_the_driver_reads(monkeypatch, world):
     assert "watchdog" not in d
 
 
+def test_dump_outputs_writes_f_after_the_timed_steps(monkeypatch, tmp_path):
+    # each stand-in iteration adds 1 to f: the dumped f_k counts warm-up + timed iterations of the main problem
+    monkeypatch.setattr(FakeProblem, "sci_iterate", lambda self, f, iters: np.asarray(f, float) + iters)
+    out = tmp_path / "dump"
+    d = _run(monkeypatch, ["--steps", "7", "--warmup", "3", "--n-per-gpu", "2048", "--dump-outputs", str(out)], 1)
+    assert d["steps"] == 7
+    f = np.load(out / "f_k.npy")
+    assert f.dtype == np.float64 and f.shape == (256,)
+    np.testing.assert_array_equal(f, 10.0)
+    assert sorted(os.listdir(out)) == ["f_k.npy"]
+
+
 @pytest.mark.parametrize("cfg", ["c1", "c2", "c4", "c5"])
 def test_single_config_lines(monkeypatch, cfg):
     d = _run(monkeypatch, ["--config", cfg], 1)

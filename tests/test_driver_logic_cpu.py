@@ -2,21 +2,15 @@
 warnings) exercised through the REAL pymbar.MBAR class on CPU.
 
 The GPU is replaced by a test-only stand-in for DeviceProblem that answers every primitive with the
-oracle, so what is tested is exactly the Python layer between pymbar.MBAR and the C ABI.  Needs the
-reference checkout (build container only); skipped elsewhere.  The stand-in lives here, not in the
+oracle, so what is tested is exactly the Python layer between pymbar.MBAR and the C ABI.  Where pymbar is not
+installed, MBAR is the stand-in of tests/_pymbar_stand_in.  The DeviceProblem stand-in lives here, not in the
 product: pymbar_b200 itself has no CPU path."""
-import os
-import sys
-
 import numpy as np
 import pytest
 
 from oracle import mbar_oracle as orc
 from tests import _cases
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HAVE_REF = os.path.isdir("/root/reference/pymbar")
-pytestmark = pytest.mark.skipif(not HAVE_REF, reason="reference checkout not present on this box")
+from tests._cases import pymbar_importable  # noqa: F401  (fixture)
 
 
 class OracleProblem:
@@ -94,9 +88,7 @@ class OracleProblem:
 
 
 @pytest.fixture()
-def patched_pymbar(monkeypatch):
-    sys.path.insert(0, os.path.join(ROOT, "oracle", "ref_shim"))
-    sys.path.insert(0, "/root/reference")
+def patched_pymbar(monkeypatch, pymbar_importable):
     import pymbar
 
     import pymbar_b200
@@ -108,8 +100,6 @@ def patched_pymbar(monkeypatch):
     pymbar_b200.install()
     yield pymbar
     pymbar_b200.uninstall()
-    sys.path.remove("/root/reference")
-    sys.path.remove(os.path.join(ROOT, "oracle", "ref_shim"))
 
 
 @pytest.mark.parametrize("name", _cases.SMALL + ["golden_example"])

@@ -8,38 +8,31 @@ import numpy as np
 import pytest
 
 from tests import _cases
+from tests._cases import pymbar_importable  # noqa: F401  (fixture)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_install_rebinds_real_pymbar_when_available():
-    if not os.path.isdir("/root/reference/pymbar"):
-        pytest.skip("reference checkout not present on this box")
-    sys.path.insert(0, os.path.join(ROOT, "oracle", "ref_shim"))
-    sys.path.insert(0, "/root/reference")
-    try:
-        import pymbar.mbar_solvers as ref_ms
+def test_install_rebinds_real_pymbar_when_available(pymbar_importable):
+    import pymbar.mbar_solvers as ref_ms
 
-        import pymbar_b200
-        from pymbar_b200 import mbar_solvers as ours
+    import pymbar_b200
+    from pymbar_b200 import mbar_solvers as ours
 
-        orig = ref_ms.solve_mbar_for_all_states
-        pymbar_b200.install()
-        assert ref_ms.solve_mbar_for_all_states is ours.solve_mbar_for_all_states
-        assert ref_ms.mbar_log_W_nk is ours.mbar_log_W_nk and ref_ms.jax_mbar_gradient is ours.mbar_gradient
-        # (MBAR.__init__ mutates the reference's module-level protocol dicts in place, mbar.py:391-406:
-        # compare the parts it never touches)
-        assert [d["method"] for d in ref_ms.DEFAULT_SOLVER_PROTOCOL] == [d["method"] for d in ours.DEFAULT_SOLVER_PROTOCOL]
-        import pymbar.mbar as mbar_mod
-        from pymbar_b200 import utils as ours_utils
+    orig = ref_ms.solve_mbar_for_all_states
+    pymbar_b200.install()
+    assert ref_ms.solve_mbar_for_all_states is ours.solve_mbar_for_all_states
+    assert ref_ms.mbar_log_W_nk is ours.mbar_log_W_nk and ref_ms.jax_mbar_gradient is ours.mbar_gradient
+    # (MBAR.__init__ mutates the reference's module-level protocol dicts in place, mbar.py:391-406:
+    # compare the parts it never touches)
+    assert [d["method"] for d in ref_ms.DEFAULT_SOLVER_PROTOCOL] == [d["method"] for d in ours.DEFAULT_SOLVER_PROTOCOL]
+    import pymbar.mbar as mbar_mod
+    from pymbar_b200 import utils as ours_utils
 
-        assert mbar_mod.kln_to_kn is ours_utils.kln_to_kn
-        pymbar_b200.uninstall()
-        assert ref_ms.solve_mbar_for_all_states is orig
-        assert mbar_mod.kln_to_kn is not ours_utils.kln_to_kn
-    finally:
-        sys.path.remove("/root/reference")
-        sys.path.remove(os.path.join(ROOT, "oracle", "ref_shim"))
+    assert mbar_mod.kln_to_kn is ours_utils.kln_to_kn
+    pymbar_b200.uninstall()
+    assert ref_ms.solve_mbar_for_all_states is orig
+    assert mbar_mod.kln_to_kn is not ours_utils.kln_to_kn
 
 
 @pytest.mark.gpu
@@ -68,14 +61,12 @@ def test_installed_backend_serves_an_mbar_like_caller():
         pymbar_b200.mbar_solvers.clear_cache()
 
 
-def test_environment_switch_installs_at_import():
+def test_environment_switch_installs_at_import(pymbar_importable):
     """PYMBAR_B200=1: importing pymbar_b200 alone rebinds pymbar.mbar_solvers (SURVEY.md section 5)."""
-    if not os.path.isdir("/root/reference/pymbar"):
-        pytest.skip("reference checkout not present on this box")
     import subprocess
 
     env = dict(os.environ, PYMBAR_B200="1", PYMBAR_DISABLE_JAX="1",
-               PYTHONPATH=os.pathsep.join([ROOT, os.path.join(ROOT, "oracle", "ref_shim"), "/root/reference"]))
+               PYTHONPATH=os.pathsep.join([ROOT] + [p for p in sys.path if p]))
     code = ("import pymbar_b200, pymbar.mbar_solvers as m, pymbar.mbar as mb; "
             "from pymbar_b200 import mbar_solvers as o; "
             "assert m.solve_mbar_for_all_states is o.solve_mbar_for_all_states; "

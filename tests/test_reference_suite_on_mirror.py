@@ -1,31 +1,18 @@
-"""The reference's own solver tests (pymbar/tests/test_mbar_solvers.py, test_mbar.py — SURVEY.md §4: the
-acceptance set for this path) run unmodified against the mirror's driver layer (device replaced by the
-oracle stand-in).  Build container only: needs /root/reference."""
-import os
-import subprocess
-import sys
-
-import pytest
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+"""The calls `pymbar.MBAR` makes while the reference's own acceptance tests run (pymbar/tests/test_mbar.py), replayed
+against the mirror's driver layer with the device replaced by the oracle stand-in: protocol chain, continuation,
+unsampled states and gauge handling of pymbar_b200.mbar_solvers must reproduce the reference's f_k and Log_W_nk
+(tests/golden/reference_suite_calls.npz, oracle/record_reference_calls.py)."""
+import pymbar_b200
+from pymbar_b200 import mbar_solvers as ms
+from tests import _cases
+from tests.test_driver_logic_cpu import OracleProblem
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/pymbar/tests"), reason="reference checkout not present")
-def test_reference_solver_tests_pass_on_the_mirror(tmp_path):
-    env = dict(os.environ)
-    env["PYTHONPATH"] = os.pathsep.join([ROOT, os.path.join(ROOT, "oracle", "ref_shim"), "/root/reference"])
-    cmd = [sys.executable, "-m", "pytest", "-q", "-p", "tests._mirror_plugin", "-p", "no:cacheprovider",
-           "/root/reference/pymbar/tests/test_mbar_solvers.py", "/root/reference/pymbar/tests/test_mbar.py",
-           # consumers of MBAR objects (FES, BAR-vs-MBAR overlap, covariance): same outcome as on the pure reference
-           # (21 passed, 8 xfailed, 4 xpassed) with the backend and the MBAR facade installed
-           "/root/reference/pymbar/tests/test_fes.py", "/root/reference/pymbar/tests/test_bar.py",
-           "/root/reference/pymbar/tests/test_covariance.py"]
-    env["PYMBAR_DISABLE_JAX"] = "1"
-    # the reference marks these tests `flaky(max_runs=2..4)` (unseeded samples, plugin absent here): same allowance
-    for _attempt in range(2):
-        out = subprocess.run(cmd, cwd=str(tmp_path), env=env, capture_output=True, text=True, timeout=1500)
-        if out.returncode == 0:
-            break
-    tail = out.stdout.strip().splitlines()[-1] if out.stdout.strip() else out.stderr[-500:]
-    assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
-    assert " passed" in tail and " failed" not in tail and " error" not in tail, tail
+def test_reference_solver_tests_pass_on_the_mirror(monkeypatch):
+    monkeypatch.setattr(ms, "DeviceProblem", OracleProblem)
+    monkeypatch.setattr(pymbar_b200._lib, "load", lambda: None)
+    monkeypatch.setenv("PYMBAR_B200_CACHE", "0")
+    calls = _cases.reference_suite_calls()
+    assert len(calls) >= 10
+    for c in calls:
+        _cases.replay_reference_suite_call(ms, c)
